@@ -2,6 +2,7 @@
 """bench.py — frames/sec of InpaintGenerator.forward on synthetic 432x240 5+3 clips (BASELINE.json metric).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--clips-per-gpu B] [--workload W]
+                    [--dump-outputs DIR]
     torchrun --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...        (N > 1, one rank per GPU, NCCL)
 
 Headline: a step = one forward over B clips per GPU (default 8 = BASELINE configs[3]'s per-GPU share: 64 clips over
@@ -24,6 +25,7 @@ import time
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True      # the tree may be read-only: the benchmark writes nothing into it
 
 import torch  # noqa: E402
 
@@ -128,6 +130,23 @@ def make_model(device, module="model.e2fgvi"):
     sd = synth_state_dict(model, "default", 0)          # the reference's own init family (BASELINE config)
     model.load_state_dict(sd, strict=True)
     return (model.to(device) if device is not None else model), sd
+
+
+DUMP_SAMPLE = 1 << 22     # elements kept of a larger output array: three arrays stay under 64 MB of float32
+
+
+def output_arrays(pred, flows):
+    """What ``model(x, l_t)`` returned, as float32 host arrays for ``--dump-outputs``.  An array of more than
+    ``DUMP_SAMPLE`` elements is replaced by ``<name>_sample``: the elements at ``DUMP_SAMPLE`` distinct flat indices
+    drawn by ``torch.randperm`` from a CPU generator seeded with 0, in increasing index order."""
+    out = {}
+    for name, t in (("pred", pred), ("flows_forward", flows[0]), ("flows_backward", flows[1])):
+        t = t.detach().float()
+        if t.numel() > DUMP_SAMPLE:
+            idx = torch.randperm(t.numel(), generator=torch.Generator().manual_seed(0))[:DUMP_SAMPLE].sort().values
+            t, name = t.reshape(-1)[idx.to(t.device)], name + "_sample"
+        out[name] = t.cpu().numpy()
+    return out
 
 
 def workload_config(name, B, world, precision="strict"):
@@ -328,7 +347,7 @@ class Measurement:
                     landed[len(landed) - 3].synchronize()
             else:
                 x = inputs[i % self.n_sets]
-            pred, _ = self.model(x, self.l_t)
+            pred, flows = self.model(x, self.l_t)
             if to_host:
                 consumed[i % 2] = torch.cuda.Event()
                 consumed[i % 2].record(main)
@@ -350,8 +369,9 @@ class Measurement:
                 download(got[self.rank * B * T:(self.rank + 1) * B * T])
         if to_host:
             main.wait_stream(d2h)                          # the timed region ends when the last result is on the host
+        return (pred, flows) if n > 0 else None
 
-    def run(self, sample_clocks=False, profile=True):
+    def run(self, sample_clocks=False, profile=True, keep_outputs=False):
         from e2fgvi_b200 import ops
         res = {}
         with torch.no_grad():
@@ -364,10 +384,12 @@ class Measurement:
             if sampler:
                 sampler.mark_start()
             e0.record()
-            self._loop(self.steps, self.dev_sets)
+            last = self._loop(self.steps, self.dev_sets)
             e1.record()
             self.sync()
             res["launches"] = ops.launch_count() - n0
+            res["outputs"] = output_arrays(*last) if keep_outputs and last else None
+            del last
             res["clocks"] = sampler.stop() if sampler else None
             ms = e0.elapsed_time(e1)
             ms_free = ms
@@ -499,6 +521,9 @@ def main():
                     help="skip the b1 / hq720 / hq1080 / video-driver sections of the default run")
     ap.add_argument("--precision", default="strict", choices=["strict", "tf32"],
                     help="library op precision (only matters for the few remaining torch glue ops)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step of the headline workload returned (rank 0) as DIR/<name>.npy, "
+                         "float32; inputs and weights are seeded, so two builds can be compared output for output")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 0)
 
@@ -529,7 +554,13 @@ def main():
     stitch_kind = ("none (one GPU)" if world == 1 else
                    "peer-memory DMA pushes + stream-memop flags (clips.PeerStitcher)" if type(head.stitch).__name__ == "PeerStitcher"
                    else "all_gather_into_tensor (clips.ClipStitcher)")
-    main_res = head.run(sample_clocks=True)
+    main_res = head.run(sample_clocks=True, keep_outputs=args.dump_outputs is not None and rank == 0)
+    if main_res["outputs"] is not None:
+        import numpy as np
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for oname, arr in main_res.pop("outputs").items():
+            np.save(os.path.join(args.dump_outputs, oname + ".npy"), arr)
+        log(f"outputs of the last timed step written to {args.dump_outputs}")
     kernels = kernel_rooflines(main_res["prof"], main_res["ms_prof"], traffic_for(name)) if rank == 0 else {}
     one_clip = head.dev_sets[0][:1].clone()
     head.free()

@@ -40,7 +40,8 @@ def _digest():
                 h.update(f.read())
     with open(os.path.join(os.path.dirname(HERE), "include", "e2fgvi_b200.h"), "rb") as f:
         h.update(f.read())
-    h.update(" ".join(NVCC_FLAGS).encode())
+    # flags without the checkout's absolute path: a built tree that is moved or copied stays up to date
+    h.update(" ".join(NVCC_FLAGS).replace(os.path.dirname(HERE), ".").encode())
     return h.hexdigest()
 
 

@@ -12,8 +12,8 @@ CPU fallback.
 * ``gen_golden.py``       the committed script that produced ``tests/golden/*.pt``.
 
 Parity pinning: the reference ships no tests or golden vectors (SURVEY §4).  The restatement is pinned against
-outputs of the reference itself run here (``tests/test_oracle_vs_reference.py`` when /root/reference exists, and
-the committed goldens everywhere).  The one third-party op on the path, ``mmcv.ops.modulated_deform_conv2d``
+outputs of the reference itself, stored as the committed goldens (``gen_golden.py``, ``gen_golden_video.py``), so the
+tests need no copy of the reference.  The one third-party op on the path, ``mmcv.ops.modulated_deform_conv2d``
 (mmcv-full 1.4.8, environment.yml:135), is NOT installable offline: its stand-in is
 ``torchvision.ops.deform_conv2d`` (same DCNv2 lineage) and the explicit restatement in ``restate.py`` matches it
 bit-for-bit on random inputs — so parity AT THE MMCV BOUNDARY IS UNPINNED against mmcv itself.

@@ -34,6 +34,8 @@ E2E_CASES = {
     "e2e_hq720_stress": (True, 720, 1296, 8, 5, "stress", 2, 7, 1, 7),
     "e2e_hq360_t16_stress": (True, 360, 648, 16, 10, "stress", 3, 8, 1, 5),
     "e2e_hq1080_t16_stress": (True, 1080, 1944, 16, 10, "stress", 4, 9, 1, 11),
+    # tests/test_oracle.py::test_oracle_vs_live_reference: a second HQ weight / frame draw, every 5th pixel
+    "e2e_hq_tiny_s3_stress": (True, 120, 216, 4, 3, "stress", 3, 9, 1, 5),
 }
 
 

@@ -85,7 +85,52 @@ def main():
             subprocess.check_call([sys.executable, child, SHIM, REFERENCE_ROOT, tmp, os.path.join(OUT, name + ".npz")]
                                   + argv, cwd=tmp)
         print(name, "done")
+    gen_network_replay()
+
+
+def gen_network_replay(name="video_hq_numref"):
+    """The reference NETWORK driven by ``oracle/restate_video.py`` on one case, for
+    ``tests/test_video.py::test_oracle_driver_bit_exact_with_reference_network``.  Written only when that run equals
+    what test.py wrote, bit for bit.  The network's output reaches the composite only as the uint8 value of each hole
+    pixel of the window's local frames (test.py:167-174), so that is what is kept, with a SHA-256 of every clip the
+    network was given."""
+    import hashlib
+    import importlib
+    import numpy as np
+    import torch
+    sys.path.insert(0, ROOT)
+    from e2fgvi_b200.synth import synth_state_dict, synth_video
+    from oracle import restate_video as RV
+    from oracle.reference_loader import reference_generator
+    model, n, h, w, family, wseed, vseed, extra = CASES[name]
+    kw = dict(num_ref=int(extra[extra.index("--num_ref") + 1]), ref_length=int(extra[extra.index("--step") + 1]),
+              neighbor_stride=int(extra[extra.index("--neighbor_stride") + 1]))
+    frames, raw = synth_video(n, h, w, vseed)
+    masks = np.stack([RV.dilate_cross(m) for m in raw])
+    ref = reference_generator(hq=model == "e2fgvi_hq")
+    ref.load_state_dict(synth_state_dict(importlib.import_module("e2fgvi_b200.model." + model).InpaintGenerator(),
+                                         family, wseed), strict=True)
+    clips, l_ts, holes = [], [], []
+    sched = RV.window_schedule(n, **kw)
+
+    def net(x, l_t):
+        i = len(clips)
+        clips.append(hashlib.sha256(x.numpy().tobytes()).hexdigest())
+        l_ts.append(l_t)
+        pred, flows = ref(x, l_t)
+        p = (((pred[:l_t, :, :h, :w] + 1) / 2).permute(0, 2, 3, 1).numpy() * 255).astype(np.uint8)
+        holes.append(p[masks[sched[i][1]].astype(bool)])
+        return pred, flows
+
+    comp = RV.finalize(RV.inpaint_video(net, frames, masks, **kw))
+    assert np.array_equal(comp, np.load(os.path.join(OUT, name + ".npz"))["comp"]), "driver != test.py"
+    np.savez_compressed(os.path.join(OUT, name + "_refnet.npz"), clip_sha256=np.array(clips), l_t=np.array(l_ts),
+                        hole_counts=np.array([len(v) for v in holes]), hole_u8=np.concatenate(holes))
+    print(name + "_refnet", len(clips), "windows", sum(len(v) for v in holes), "hole pixels")
 
 
 if __name__ == "__main__":
-    main()
+    if "--network-replay-only" in sys.argv:
+        gen_network_replay()
+    else:
+        main()

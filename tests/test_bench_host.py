@@ -67,3 +67,20 @@ def test_clock_sampler_keeps_only_samples_of_the_timed_region():
     s.p = FakeProc([f"Tue Sep 23 13:20:46 2026, 1700, 1965, {capped}"])   # unknown timestamp format: kept
     s.t0 = now - 0.5
     assert s.stop() == {"sm_mhz": 1700.0, "sm_max_mhz": 1965.0, "samples": 1, "reasons": ["sw_power_cap"]}
+
+
+def test_dump_outputs_keep_small_arrays_and_sample_large_ones():
+    """--dump-outputs: float32 arrays, small ones whole, a large one as the same seeded sample of distinct elements on
+    every run, three sampled arrays within 64 MB."""
+    import numpy as np
+    import torch
+
+    import bench
+    assert 3 * bench.DUMP_SAMPLE * 4 <= 64 << 20
+    pred = torch.arange(bench.DUMP_SAMPLE + 1000, dtype=torch.float32)     # value == flat index
+    flows = (torch.ones(2, 3), torch.zeros(2, 3, dtype=torch.float64))
+    a, b = bench.output_arrays(pred, flows), bench.output_arrays(pred, flows)
+    assert sorted(a) == ["flows_backward", "flows_forward", "pred_sample"]
+    assert all(v.dtype == np.float32 for v in a.values()) and a["flows_forward"].shape == (2, 3)
+    s = a["pred_sample"]
+    assert s.shape == (bench.DUMP_SAMPLE,) and np.array_equal(s, b["pred_sample"]) and np.all(np.diff(s) > 0)
