@@ -66,6 +66,8 @@ SIGNATURES = {
     "e2f_video_compose": (_i, [_fp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _vp]),
     "e2f_video_blend": (_i, [_vp, _vp, _vp, _fp, _i, _c.c_int64, _vp]),
     "e2f_video_finalize": (_i, [_fp, _vp, _c.c_int64, _vp]),
+    "e2f_psnr_ssim_workspace_bytes": (_c.c_size_t, [_i, _i, _i, _i]),
+    "e2f_psnr_ssim": (_i, [_vp, _fp, _vp, _vp, _i, _i, _i, _i, _c.c_double, _vp, _vp]),
     "e2f_launch_count": (_c.c_int64, []),
 }
 

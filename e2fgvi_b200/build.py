@@ -13,7 +13,7 @@ CSRC = os.path.join(HERE, "csrc")
 LIB_PATH = os.path.join(HERE, "libe2fgvi_b200.so")
 STAMP = LIB_PATH + ".stamp"
 
-SOURCES = ["api.cu", "flow_warp.cu", "dcn.cu", "focal_attn.cu", "t2t.cu", "gemm.cu", "conv.cu", "elementwise.cu", "video.cu", "spynet.cu", "conv_kxn.cu", "peer.cu"]
+SOURCES = ["api.cu", "flow_warp.cu", "dcn.cu", "focal_attn.cu", "t2t.cu", "gemm.cu", "conv.cu", "elementwise.cu", "video.cu", "spynet.cu", "conv_kxn.cu", "peer.cu", "metrics.cu"]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a",
     "-O3", "-lineinfo", "-std=c++17",

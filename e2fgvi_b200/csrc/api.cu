@@ -479,4 +479,28 @@ int e2f_video_finalize(const float* comp, uint8_t* out, int64_t count, void* str
   return finish(launch_video_finalize(comp, out, static_cast<long long>(count), static_cast<cudaStream_t>(stream)), "e2f_video_finalize");
 }
 
+static int psnr_ssim_shape_checks(const char* who, int n, int h, int w, int win_size) {
+  if (n <= 0 || h <= 0 || w <= 0) { set_error("%s: bad shape n=%d h=%d w=%d", who, n, h, w); return E2F_ERR_BAD_ARG; }
+  if (win_size < 3 || !(win_size & 1)) { set_error("%s: win_size %d must be odd and >= 3", who, win_size); return E2F_ERR_BAD_ARG; }
+  if (win_size > h || win_size > w) { set_error("%s: win_size %d exceeds the image side (h=%d w=%d)", who, win_size, h, w); return E2F_ERR_BAD_ARG; }
+  if (win_size > psnr_ssim_max_win()) { set_error("%s: win_size %d > %d unsupported", who, win_size, psnr_ssim_max_win()); return E2F_ERR_UNSUPPORTED; }
+  return 0;
+}
+
+size_t e2f_psnr_ssim_workspace_bytes(int n, int h, int w, int win_size) {
+  if (psnr_ssim_shape_checks("e2f_psnr_ssim_workspace_bytes", n, h, w, win_size)) return 0;
+  return psnr_ssim_workspace_bytes(n, h, w, win_size);
+}
+
+int e2f_psnr_ssim(const uint8_t* ref, const float* test, double* psnr, double* ssim, int n, int h, int w, int win_size,
+                  double data_range, void* workspace, void* stream) {
+  const char* who = "e2f_psnr_ssim";
+  if (!ref || !test || !psnr || !ssim || !workspace) { set_error("%s: null pointer", who); return E2F_ERR_BAD_ARG; }
+  const int st = psnr_ssim_shape_checks(who, n, h, w, win_size);
+  if (st) return st;
+  if (!(data_range > 0.0)) { set_error("%s: data_range must be positive", who); return E2F_ERR_BAD_ARG; }
+  if (!aligned(test, 4) || !aligned(psnr, 8) || !aligned(ssim, 8) || !aligned(workspace, 8)) { set_error("%s: test needs 4-byte, psnr / ssim / workspace 8-byte alignment", who); return E2F_ERR_ALIGNMENT; }
+  return finish(launch_psnr_ssim(ref, test, psnr, ssim, n, h, w, win_size, data_range, workspace, static_cast<cudaStream_t>(stream)), who);
+}
+
 }  // extern "C"

@@ -117,4 +117,9 @@ int launch_video_blend(const uint8_t* img, const int* ids, const int* first, flo
                        long long frame_elems, cudaStream_t stream);
 int launch_video_finalize(const float* comp, uint8_t* out, long long count, cudaStream_t stream);
 
+size_t psnr_ssim_workspace_bytes(int n, int h, int w, int win);
+int psnr_ssim_max_win();
+int launch_psnr_ssim(const uint8_t* ref, const float* test, double* psnr, double* ssim, int n, int h, int w, int win,
+                     double data_range, void* workspace, cudaStream_t stream);
+
 }  // namespace e2f

@@ -140,3 +140,40 @@ def synth_video(n, h, w, seed=0):
         x0 = int((w - ww) * (i / max(n - 1, 1)))
         masks[i, y0:y0 + hh, x0:x0 + ww] = 1
     return frames, masks
+
+
+def write_eval_dataset(root, videos, h=270, w=480, seed=0, dataset="davis"):
+    """A synthetic dataset in the layout the reference's evaluate.py reads (core/dataset.py:82-135):
+    ``<root>/<dataset>/test.json``, ``JPEGImages/<name>.zip`` of JPEG frames and ``test_masks/<name>/%05d.png``.
+    ``videos`` is ``[(name, n_frames)]``.  Frames are smooth drifting colour waves at ``h`` x ``w`` (not 432x240, so
+    the loader's resize matters); holes are a moving rectangle, and zip members are written out of order so the
+    loader's sort matters.  Deterministic for a given seed, OpenCV and Pillow."""
+    import json
+    import os
+    import zipfile
+    import cv2
+    import numpy as np
+    base = os.path.join(root, dataset)
+    os.makedirs(os.path.join(base, "JPEGImages"), exist_ok=True)
+    yy = np.linspace(0, 1, h, dtype=np.float64)[:, None, None]
+    xx = np.linspace(0, 1, w, dtype=np.float64)[None, :, None]
+    for v, (name, n) in enumerate(videos):
+        rng = np.random.default_rng([seed, v])
+        ph = rng.uniform(0, 6.28, size=3)
+        os.makedirs(os.path.join(base, "test_masks", name), exist_ok=True)
+        with zipfile.ZipFile(os.path.join(base, "JPEGImages", f"{name}.zip"), "w") as z:
+            for i in reversed(range(n)):
+                img = 0.5 + 0.35 * np.sin(6.28 * (1.3 * xx + 0.7 * yy + 0.02 * i) + ph) * np.cos(6.28 * (0.9 * yy - 0.015 * i))
+                ok, jpg = cv2.imencode(".jpg", cv2.cvtColor((img * 255).round().astype(np.uint8), cv2.COLOR_RGB2BGR))
+                assert ok
+                z.writestr(f"{i:05d}.jpg", jpg.tobytes())
+        hh, ww = h // 6, w // 8
+        for i in range(n):
+            m = np.zeros((h, w), np.uint8)
+            y0 = int((h - hh) * (0.5 + 0.4 * math.sin(0.5 * i + v)))
+            x0 = int((w - ww) * (i / max(n - 1, 1)))
+            m[y0:y0 + hh, x0:x0 + ww] = 255
+            cv2.imwrite(os.path.join(base, "test_masks", name, f"{i:05d}.png"), m)
+    with open(os.path.join(base, "test.json"), "w") as f:
+        json.dump({name: n for name, n in videos}, f)
+    return root

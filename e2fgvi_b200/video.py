@@ -131,6 +131,13 @@ class VideoInpainter:
 
     @torch.no_grad()
     def __call__(self, frames, masks, device=None):
+        """-> (N,H,W,3) uint8 on the device: the frames test.py writes (test.py:195)."""
+        return finalize(self.composite(frames, masks, device))
+
+    @torch.no_grad()
+    def composite(self, frames, masks, device=None):
+        """-> (N,H,W,3) fp32 on the device: the blended canvas before the final uint8 truncation, which is what
+        evaluate.py scores (evaluate.py:113-114,125-126)."""
         device = torch.device(device) if device is not None else (
             frames.device if frames.is_cuda else torch.device("cuda", torch.cuda.current_device()))
         if frames.dtype != torch.uint8 or masks.dtype != torch.uint8:
@@ -177,4 +184,4 @@ class VideoInpainter:
             for i in nb:
                 seen[i] = True
         assert all(seen), "every frame is a neighbour of some window (test.py:147-150)"
-        return finalize(comp)
+        return comp

@@ -388,6 +388,20 @@ int e2f_video_blend(const uint8_t* img, const int* ids, const int* first, float*
                     void* stream);
 int e2f_video_finalize(const float* comp, uint8_t* out, int64_t count, void* stream);
 
+/* Per-frame PSNR and SSIM of evaluate.py (core/metrics.py:20-53: calculate_psnr, and scikit-image 0.16
+ * compare_ssim(ref, test, data_range, multichannel=True, win_size) with scipy's uniform window), in fp64.
+ *   ref  [N][H][W][3] uint8 (the original frames), test [N][H][W][3] fp32 (the canvas), psnr / ssim [N] fp64.
+ *   psnr[f] = 20 log10(data_range / sqrt(mean((ref - test)^2))), +inf when the frames are equal;
+ *   ssim[f] = mean over the 3 channels and over the outputs whose win_size x win_size window lies inside the frame
+ *             of skimage's S, with C1 = (0.01 data_range)^2, C2 = (0.03 data_range)^2 and sample covariances.
+ * win_size must be odd, >= 3 and <= min(H, W) (skimage raises ValueError otherwise), and <= 255 (E2F_ERR_UNSUPPORTED).
+ * `workspace` is device memory of at least e2f_psnr_ssim_workspace_bytes(n, h, w, win_size) bytes, 8-byte aligned;
+ * a smaller one is not detected.  e2f_psnr_ssim_workspace_bytes returns 0 for arguments e2f_psnr_ssim rejects.
+ * Deterministic: a frame's result does not depend on the other frames of the call, and no atomics are used. */
+size_t e2f_psnr_ssim_workspace_bytes(int n, int h, int w, int win_size);
+int e2f_psnr_ssim(const uint8_t* ref, const float* test, double* psnr, double* ssim, int n, int h, int w, int win_size,
+                  double data_range, void* workspace, void* stream);
+
 /* Number of kernel launches issued through this library since load (all threads); used by bench.py's
  * "gpu_launches" accounting. */
 int64_t e2f_launch_count(void);
